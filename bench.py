@@ -421,7 +421,7 @@ def run_c1(args, w, wname):
         for _ in range(max(args.warmup, 3)):
             call()
         ts = []
-        for _ in range(max(args.steps, 10)):
+        for _ in range(args.steps):
             t0 = time.perf_counter()
             g, p, L = call()
             ts.append(time.perf_counter() - t0)
@@ -451,7 +451,7 @@ def run_c1(args, w, wname):
 
     evs = []
     l0 = None
-    for i in range(3 + max(args.steps, 10)):        # production configuration: no per-kernel events, the run replayed as a CUDA graph
+    for i in range(3 + args.steps):                 # production configuration: no per-kernel events, the run replayed as a CUDA graph
         if i == 3:
             torch.cuda.synchronize()
             l0 = vb.launches
@@ -462,6 +462,8 @@ def run_c1(args, w, wname):
         if i >= 3:
             evs.append((e0, e1))
     torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, g_d, p_d, out, S)
     res_ms = float(np.median([a.elapsed_time(b) for a, b in evs]))
     n_steps = len(evs)
     launches = (vb.launches - l0) / n_steps
@@ -516,6 +518,32 @@ def load_peaks():
     return 6650.0, 'fallback 6.65 TB/s (B200_PROFILING.md)'
 
 
+DUMP_BYTES, DUMP_GAMMA_BYTES = 60 << 20, 32 << 20         # 60 MiB of payload + .npy headers stay under 64 MB
+
+
+def dump_outputs(directory, gamma, pi, out, S, trace=None):
+    """Write what the last timed step returned to its caller as DIR/<name>.npy (float32 / float64), for comparing two
+    builds output for output: pi [B,S], Li, n_iters, flags (and the batch ELBO trace) in full, and the responsibilities
+    gamma [N,S] for a fixed, seeded sample of frames (rows of the packed array, row indices alongside): at most 32 MB
+    of gamma and 64 MB in all."""
+    import torch
+    arrays = {'pi': pi[:, :S].float(), 'Li': out['Li'].double(), 'n_iters': out['n_iters'].double(),
+              'flags': out['flags'].double()}
+    if trace is not None:
+        arrays['elbo_trace'] = torch.as_tensor(np.asarray(trace, dtype=np.float64))
+    rest = sum(a.numel() * a.element_size() for a in arrays.values())
+    if rest > DUMP_BYTES // 2:
+        raise SystemExit(f'--dump-outputs: the per-recording outputs alone take {rest} bytes')
+    N = gamma.shape[0]
+    k = min(N, DUMP_GAMMA_BYTES // (4 * S), (DUMP_BYTES - rest) // (4 * S + 8))
+    rows = np.sort(np.random.default_rng(0).choice(N, size=k, replace=False))
+    arrays['gamma_sample'] = gamma[torch.from_numpy(rows).to(gamma.device), :S].float()
+    arrays['gamma_sample_rows'] = torch.from_numpy(rows.astype(np.float64))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + '.npy'), a.cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -537,7 +565,16 @@ def main():
                     help="what feeds the EM loop: 'project' = rho = X.V (the headline definition, SURVEY 8d); 'xvectors' = the "
                          "real-data chain vbx_prepare_xvectors (x-vector transform + PLDA projection, two tcgen05 passes)")
     ap.add_argument('--extra', default='', help='comma separated extra workloads to time (kernel-only) in the same run')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (the inputs are seeded: the same '
+                         'arguments give the same inputs, so two builds can be compared output for output).  With '
+                         'several ranks, rank 0 writes its own recordings (gamma, pi, Li, n_iters, flags) and the '
+                         'batch-wide elbo_trace')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the device path (--impl b200)')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     w, wname = WORKLOADS[args.workload], args.workload
     if args.impl == 'reference':
@@ -681,7 +718,7 @@ def main():
         launches = (vb.launches - l0) / steps
         tr = trace.cpu().numpy()          # batch-wide ELBO trace of the last timed step (all ranks, in-library all-reduce)
         # ---- kernel pass: 3 steps with per-kernel CUDA events on ONE stream, direct launches ----
-        gamma_keep, pi_keep, out_keep = gamma.clone(), pi.clone(), {k: v.clone() for k, v in out.items() if k in ('Li', 'n_iters')}
+        gamma_keep, pi_keep, out_keep = gamma.clone(), pi.clone(), {k: v.clone() for k, v in out.items() if k in ('Li', 'n_iters', 'flags')}
         if partitioned:
             serial = VbxBatch(lengths, R_DIM, w['S'], device=device, fb_split=args.fb_split)
             configure(serial, timing=True)
@@ -744,6 +781,8 @@ def main():
 
     res = time_workload(w, wname, args.steps, args.warmup, with_clocks=True)
     dbg(f'timed region done: {res["ms"]:.3f} ms/step')
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res['gamma'], res['pi'], res['out'], w['S'], trace=res['trace'])
     ms, N, N_total = res['ms'], res['N'], res['N_total']
     value = N_total / (ms / 1e3)
 

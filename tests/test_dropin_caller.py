@@ -1,7 +1,7 @@
 """The reference's real caller against the drop-in: `python VBx/vbhmm.py ...` unchanged (run_example.sh:23-34,
 VBx/vbhmm.py:45,154-158), started through the launcher that makes `from VBx import VBx` resolve to vbx_b200.
 
-The reference tree exists only in the build container (no GPU there); the GPU box has no reference tree.  So:
+The original VBx is not part of this repository; the tests that execute it read a checkout named by $VBX_REF.  So:
   * the import mechanics are tested everywhere with a two-directory mock (no GPU, no reference needed);
   * the unchanged vbhmm.py is executed where the reference exists: with a GPU it must reproduce exp/ES2005a.rttm, without
     one it must get through the reference's own I/O + AHC stages and then fail LOUDLY inside the drop-in (no CPU fallback);
@@ -15,15 +15,15 @@ import textwrap
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get('VBX_REF', '/root/reference')
+REF = os.environ.get('VBX_REF', '')
 SHIMS = os.path.join(ROOT, 'tests', 'shims')
 GOLD = os.path.join(ROOT, 'tests', 'golden')
 
 
 def reference_script():
-    """The unmodified vbhmm.py: the reference tree (build container) or the pip-installed copy under baseline/_ref (it
-    travels to the GPU box; installed with `pip install --target baseline/_ref` from /root/reference, see DESIGN.md)."""
-    for d in (os.path.join(REF, 'VBx'), os.path.join(ROOT, 'baseline', '_ref', 'VBx')):
+    """The unmodified vbhmm.py: a checkout of the original VBx named by $VBX_REF, or a copy installed with
+    `pip install --target baseline/_ref` from one (see DESIGN.md)."""
+    for d in ([os.path.join(REF, 'VBx')] if REF else []) + [os.path.join(ROOT, 'baseline', '_ref', 'VBx')]:
         if os.path.isfile(os.path.join(d, 'vbhmm.py')) and os.path.isfile(os.path.join(d, 'VBx.py')):
             return os.path.join(d, 'vbhmm.py')
     return None
@@ -69,7 +69,7 @@ def test_shadow_module_exports_the_reference_names():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(reference_script() is None, reason='no copy of the reference (reference tree or baseline/_ref)')
+@pytest.mark.skipif(reference_script() is None, reason='no copy of the original VBx ($VBX_REF or baseline/_ref)')
 def test_unchanged_vbhmm_py_on_the_gpu_from_fixture_inputs(tmp_path):
     """On the GPU box: the UNCHANGED vbhmm.py (pip-installed copy of the reference) through the launcher, with its input
     files rebuilt from the reference-generated fixtures (x-vector ark, segments, binary Kaldi PLDA, transform) - the
@@ -105,7 +105,8 @@ def test_unchanged_vbhmm_py_on_the_gpu_from_fixture_inputs(tmp_path):
     assert len(set(mapping.values())) == len(mapping)
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, 'VBx', 'vbhmm.py')), reason='reference tree not present')
+@pytest.mark.skipif(not REF or not os.path.isfile(os.path.join(REF, 'VBx', 'vbhmm.py')),
+                    reason='set VBX_REF to a checkout of the original VBx (its exp/ inputs are needed)')
 def test_unchanged_vbhmm_py_through_the_dropin(tmp_path):
     import torch
     from vbx_b200 import formats

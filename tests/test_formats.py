@@ -110,9 +110,10 @@ def test_transform_h5_rejects_other_files(tmp_path):
 
 
 def test_shipped_model_files_when_present():
-    ref_dir = '/root/reference/VBx/models/ResNet101_16kHz'
-    if not os.path.exists(ref_dir):
-        pytest.skip('reference model files only exist in the build container')
+    """The readers on the model files shipped with the original VBx (a checkout named by $VBX_REF)."""
+    ref_dir = os.path.join(os.environ.get('VBX_REF', ''), 'VBx', 'models', 'ResNet101_16kHz')
+    if not os.environ.get('VBX_REF') or not os.path.exists(ref_dir):
+        pytest.skip('set VBX_REF to a checkout of the original VBx to read its model files')
     m = np.load(os.path.join(ROOT, 'tests', 'golden', 'es2005a_model.npz'))
     mean1, mean2, lda = formats.read_xvec_transform(os.path.join(ref_dir, 'transform.h5'))
     np.testing.assert_array_equal(mean1, m['mean1'])

@@ -46,17 +46,19 @@ def test_soft_init_and_hard_labels_cpu(es):
 
 
 def test_xvector_transform_matches_reference_cpu(es):
-    """VBx/vbhmm.py:129 (float64, CPU tensors here; the same code runs on the device)."""
-    from vbx_b200 import formats
-    ref_dir = '/root/reference/VBx/models/ResNet101_16kHz'
-    if not os.path.exists(ref_dir):
-        pytest.skip('reference model files only exist in the build container')
-    mean1, mean2, lda = formats.read_xvec_transform(os.path.join(ref_dir, 'transform.h5'))
-    x = pipeline.xvector_transform(torch.from_numpy(es['x_raw'].astype(np.float64)), torch.from_numpy(mean1),
-                                   torch.from_numpy(mean2), torch.from_numpy(lda))
+    """VBx/vbhmm.py:129 (float64, CPU tensors here; the same code runs on the device), on the shipped ResNet101_16kHz
+    model as stored in es2005a_model.npz.  Its PLDA is stored diagonalised (VBx/vbhmm.py:107-113: psi descending).
+    The diagonalisation sees the model only through W = (tr' tr)^-1 and B = (tr' psi^-1 tr)^-1, which a permutation
+    and sign flips of the rows of tr (with psi permuted alike) leave unchanged: from such a model it must recover the
+    reference's order, signs and features."""
+    m = np.load(os.path.join(GOLD, 'es2005a_model.npz'))
+    assert str(m['sha_plda']) == str(es['sha_plda']) and str(m['sha_transform']) == str(es['sha_transform'])
+    x = pipeline.xvector_transform(torch.from_numpy(es['x_raw'].astype(np.float64)), torch.from_numpy(m['mean1']),
+                                   torch.from_numpy(m['mean2']), torch.from_numpy(m['lda']))
     np.testing.assert_allclose(x.numpy(), es['x_lda'], atol=1e-12)
-    mu, tr, psi = formats.read_kaldi_plda(os.path.join(ref_dir, 'plda'))
-    mu, tr, psi = pipeline.diagonalise_plda(mu, tr, psi)
+    rng = np.random.default_rng(0)
+    perm, sign = rng.permutation(len(m['plda_psi'])), rng.choice([-1.0, 1.0], size=len(m['plda_psi']))
+    mu, tr, psi = pipeline.diagonalise_plda(m['plda_mu'], sign[:, None] * m['plda_tr'][perm], m['plda_psi'][perm])
     fea = pipeline.plda_project(x, torch.from_numpy(mu), torch.from_numpy(tr), 128)
     np.testing.assert_allclose(fea.numpy(), es['fea'], atol=1e-9)
     np.testing.assert_allclose(psi[:128], es['Phi'], rtol=1e-12)
